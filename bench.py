@@ -16,6 +16,9 @@ A "step" = one pass of the hot path over one batch of R requests per GPU:
            box's host cores, same workload.
 `--impl reference` times that CPU port alone (all host threads) with the same JSON contract.
 `--workload E` runs BASELINE.json's last configuration (1M requests x 4096 endpoints, request-sharded over the N GPUs).
+`--dump-outputs DIR` writes what the last timed step returned to its caller (pick, pick_score, tie_count) as DIR/<name>.npy
+           in float64 (DIR/<name>_rank<r>.npy per rank on N > 1); the inputs are seeded, so two builds run with the same
+           arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -120,6 +123,13 @@ def time_oracle(o, osnap, prof, idx, seed, wset, R, n_threads, min_seconds=2.0, 
     return float(np.median(times)), len(times)
 
 
+def dump_outputs(path, arrays):
+    """--dump-outputs: one float64 .npy per array (int32 picks and tie counts are exact in float64)."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def host_cpus():
     """What the box really offers the CPU arm: logical CPUs, the affinity mask and the cgroup CPU quota (a container may see
     128 CPUs and be allowed ten of them)."""
@@ -180,7 +190,7 @@ def run_reference(args):
     cores = os.cpu_count() or 1
 
     def step(threads=cores, n=R):
-        oracle_batch(o, osnap, prof, idx, seed, sets[0], n, threads)
+        return oracle_batch(o, osnap, prof, idx, seed, sets[0], n, threads)
 
     threads, tried = best_thread_count(step, R, cores)
     for _ in range(args.warmup):
@@ -188,8 +198,10 @@ def run_reference(args):
     times = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        step(threads)
+        res = step(threads)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: res[k] for k in ("pick", "pick_score", "tie_count")})
     med = float(np.median(times))
     value = R / med
     n1 = 4096
@@ -271,8 +283,7 @@ def run_gpu(args):
     import torch.distributed as dist
 
     import _pkg
-    _pkg.load_build().build()
-    pkg = _pkg.load()
+    pkg = _pkg.load()   # the library __graft_entry__.build() made; bench.py compiles nothing and writes nothing in the tree
     import importlib
     sharding = importlib.import_module(_pkg.NAME + ".sharding")   # the multi-GPU host helpers (commit-stream exchange)
 
@@ -447,6 +458,9 @@ def run_gpu(args):
     barrier()
     ms_max = allreduce(e0.elapsed_time(e1), RMAX)
     value = world * R * args.steps / (ms_max * 1e-3)
+    if args.dump_outputs:
+        sfx = f"_rank{rank}" if world > 1 else ""
+        dump_outputs(args.dump_outputs, {k + sfx: v.cpu().numpy() for k, v in out.items()})
     # the timed steps must still produce oracle-exact picks on every rank (last step used set (warmup+steps-1)%NSETS)
     check_parity((args.warmup + args.steps - 1) % NSETS, 2048, "timed region")
 
@@ -1059,7 +1073,11 @@ def main():
     ap.add_argument("--dev-split", type=int, default=None, help="experiment: slices per device-resident batch (engine debug key 5)")
     ap.add_argument("--dev-streams", type=int, default=None, help="experiment: streams the slices alternate over (engine debug key 6)")
     ap.add_argument("--quick", action="store_true", help="skip the side legs (per-kernel timing, §8f profiles, CPU baselines)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (pick, pick_score, tie_count) as DIR/<name>.npy in float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     set_workload(args.workload, int(os.environ.get("WORLD_SIZE", "1")))
